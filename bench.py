@@ -2,6 +2,7 @@
 """bench.py — the contract benchmark of the attention + FusedMLP hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2] [--no-secondary]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input at the Llama-2-7B layer shapes of
 BASELINE.json configs[2] (the configuration the metric's "SwiGLU-MLP" is quoted on and the largest single-GPU one):
@@ -439,6 +440,30 @@ def build_step(cx, w, args):
     return step, st
 
 
+DUMP_ROWS = 1024  # token rows kept per output: the C3 step's two [T, 4096] outputs come to 32 MB as float32
+
+
+def dump_outputs(cx, st, out_dir):
+    """Write what the last timed step computed as float32 .npy files: ``attn_out`` (the attention output O as
+    [tokens, Hq*D]) and ``mlp_out`` (the MLP output y as [tokens, h]). Both keep the same DUMP_ROWS token rows, drawn
+    with a fixed seed, so two builds run with the same arguments can be compared element for element."""
+    import numpy as np
+    torch = cx.torch
+    T = st["T"]
+    rows = np.sort(np.random.default_rng(0).choice(T, size=min(T, DUMP_ROWS), replace=False))
+    idx = torch.from_numpy(rows).to(cx.dev)
+    o = st["o"].reshape(T, -1).index_select(0, idx)
+    if cx.world > 1:  # every rank holds Hq/N heads: put the job's heads side by side, rank order
+        parts = [torch.empty_like(o) for _ in range(cx.world)]
+        cx.dist.all_gather(parts, o)
+        o = torch.cat(parts, dim=1)
+    y = st["y"].reshape(T, -1).index_select(0, idx)
+    if cx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "attn_out.npy"), o.float().cpu().numpy())
+        np.save(os.path.join(out_dir, "mlp_out.npy"), y.float().cpu().numpy())
+
+
 def e2e_leg(cx, w, st, args):
     """End to end through the public nn.Module API with pinned HOST buffers: every step copies its inputs host -> device
     and its results device -> host inside the timed region (three streams, double-buffered device tensors)."""
@@ -759,6 +784,8 @@ def run_ours(args, w):
         for b in pool["bufs"]:
             b.check()
     elapsed_ms, fa_ms, mlp_ms = cx.max_over_ranks([elapsed_ms, fa_ms, mlp_ms])
+    if args.dump_outputs:
+        dump_outputs(cx, st, args.dump_outputs)
 
     e2e = e2e_leg(cx, w, st, args)
     breakdown = tp_breakdown_leg(cx, w, st, args) if n > 1 else None
@@ -870,7 +897,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-ring", action="store_true")
     ap.add_argument("--group-rows", type=int, default=0, help="override the GEMM L2 raster group (rows)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (a fixed row sample) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -1,8 +1,8 @@
-"""Generate golden input/output vectors by RUNNING THE REFERENCE in the authoring container.
+"""Generate golden input/output vectors by RUNNING THE REFERENCE (the original project) on CPU.
 
-    python tests/golden/make_golden.py            # needs /root/reference (read-only); writes tests/golden/*.pt
+    B200_REFERENCE_DIR=<checkout of the reference> python tests/golden/make_golden.py   # writes tests/golden/*.pt
 
-The reference cannot travel to the GPU box, so the vectors are committed. What is runnable in the reference
+The reference is not part of this repository, so the vectors are committed. What is runnable in the reference
 (SURVEY.md §0):
   * kernels/mlp/fused_mlp.py — FusedTransformerMLP / FusedMLP* forward (always the eager path, F5)
   * kernels/triton/mlp_kernels.py:759 pytorch_fused_mlp
@@ -10,7 +10,7 @@ The reference cannot travel to the GPU box, so the vectors are committed. What i
     only when ``import triton`` fails (F8); we mask triton in sys.modules to reach it. Causal vectors use the
     finite -1e9 additive mask the reference's FA kernels use (flash_attention_kernels.py:253).
   * parallelism/sequence_parallel.py:480-517 SequenceParallelAttention._local_attention (eager softmax attention)
-Everything is seeded; tensors are small (fp32) so the fixture stays a few hundred KB.
+Everything is seeded; tensors are small (fp32) so every fixture file stays under 1 MB.
 """
 from __future__ import annotations
 
@@ -21,7 +21,7 @@ import types
 
 import torch
 
-REF = os.environ.get("B200_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("B200_REFERENCE_DIR", "")
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -120,12 +120,45 @@ def attention_vectors():
     y = sp.SequenceParallelAttention._local_attention(stub, q, k, v, pad)
     out["sp_local_attention_padmask"] = {"q": q, "k": k, "v": v, "mask": pad, "kv_lens": torch.tensor([S, 150]),
                                          "y": y.clone()}
+    return keep_heads(out, ATTN_KEPT_HEADS)
+
+
+# Attention is independent per (batch, head): the vectors are generated at H=4 (so the seeded inputs stay the ones first
+# generated) and only these heads are stored, which keeps the file under 1 MB.
+ATTN_KEPT_HEADS = [0]
+
+
+def keep_heads(vecs, heads):
+    """The attention vectors restricted to ``heads``: q/k/v/y [B,H,S,D] (ring fallback y [B,S,H*D]) sliced on the head
+    axis into compact storage; tensors shared between entries stay shared so that torch.save writes them once."""
+    idx = torch.tensor(heads)
+    sliced = {}
+
+    def head_slice(t):
+        if id(t) not in sliced:
+            sliced[id(t)] = t.index_select(1, idx).contiguous()
+        return sliced[id(t)]
+
+    out = {}
+    for name, d in vecs.items():
+        e = dict(d)
+        for n in ("q", "k", "v"):
+            e[n] = head_slice(d[n])
+        y = d["y"]
+        if name.startswith("ring_fallback"):  # [B, S, H*D] -> [B, S, len(heads)*D]
+            B, S, _ = y.shape
+            D = d["q"].shape[-1]
+            e["y"] = y.view(B, S, -1, D).index_select(2, idx).reshape(B, S, len(heads) * D).contiguous()
+        else:
+            e["y"] = y.index_select(1, idx).contiguous()
+        out[name] = e
     return out
 
 
 def main():
     if not os.path.isdir(REF):
-        raise SystemExit(f"{REF} not found: golden vectors can only be regenerated where the reference is mounted")
+        raise SystemExit(f"B200_REFERENCE_DIR={REF!r} is not a directory: golden vectors can only be regenerated from a "
+                         "checkout of the reference")
     sys.path.insert(0, REF)
     torch.set_num_threads(1)
     torch.use_deterministic_algorithms(True)
