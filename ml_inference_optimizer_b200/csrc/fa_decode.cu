@@ -55,8 +55,8 @@ struct Params {
 template <int D, int G, typename T, bool PAGED>
 __global__ void __launch_bounds__(NUM_THREADS, 2)
 decode_kernel(const Params p) {
-  // 16-byte loads in flight per lane for K (and again for V); fewer for wide GQA groups so that two CTAs fit per SM
-  constexpr int NLOAD = (G >= 4) ? 4 : 8;
+  // 16-byte loads in flight per lane for K (and again for V); G is 1 or 2 here (wider groups run decode_gqa_mma_kernel)
+  constexpr int NLOAD = 8;
   constexpr int LPR = D / 8;          // lanes per KV row
   constexpr int RPW = 32 / LPR;       // rows per warp-wide load
   constexpr int TILE = NLOAD * RPW;   // keys per warp iteration
@@ -737,8 +737,6 @@ int dispatch_group(int G, const Params& p, bool paged, cudaStream_t stream) {
   switch (G) {
     case 1: return launch_decode<D, 1, T>(p, paged, stream);
     case 2: return launch_decode<D, 2, T>(p, paged, stream);
-    case 4: return launch_decode<D, 4, T>(p, paged, stream);
-    case 8: return launch_decode<D, 8, T>(p, paged, stream);
     default:
       return set_error(B200_ERR_UNSUPPORTED, "decode: Hq/Hkv = %d is not supported (1 .. 16)", G);
   }

@@ -25,7 +25,8 @@ import torch
 
 __all__ = [
     "attention_ref", "decode_attention_ref", "paged_gather", "kv_append_ref", "lse_merge_ref", "mlp_ref",
-    "linear_act_ref", "layernorm_ref", "gelu_tanh", "rel_err_percent", "max_abs_err", "ring_attention_ref", "tp_mlp_ref",
+    "linear_act_ref", "layernorm_ref", "gelu_tanh", "rel_err_percent", "max_abs_err", "tile_errors", "ring_attention_ref",
+    "tp_mlp_ref",
 ]
 
 
@@ -39,6 +40,46 @@ def rel_err_percent(a: torch.Tensor, b: torch.Tensor) -> float:
 
 def max_abs_err(a: torch.Tensor, b: torch.Tensor) -> float:
     return float((a.double() - b.double()).abs().max())
+
+
+def _tiles(t: torch.Tensor, tiling: str, hkv: Optional[int], tile: int) -> torch.Tensor:
+    """``t`` regrouped as [num_tiles, elements]; ragged edges are zero-padded (zeros add nothing to either sum or max)."""
+    if tiling == "attn":                                   # [B,S,H,D]: one tile per (b, h, `tile` query rows)
+        B, S, H, D = t.shape
+        t = torch.nn.functional.pad(t, (0, 0, 0, 0, 0, (-S) % tile))
+        return t.view(B, -1, tile, H, D).permute(0, 3, 1, 2, 4).reshape(-1, tile * D)
+    if tiling == "decode":                                 # [B,Hq,D]: one tile per (b, kv head) = the G query heads it serves
+        B, Hq, D = t.shape
+        return t.reshape(B * hkv, (Hq // hkv) * D)
+    if tiling == "2d":                                     # [T,N]: one tile per `tile` x `tile` block
+        t = t.reshape(-1, t.shape[-1])
+        T, N = t.shape
+        t = torch.nn.functional.pad(t, (0, (-N) % tile, 0, (-T) % tile))
+        return t.view(t.shape[0] // tile, tile, t.shape[1] // tile, tile).permute(0, 2, 1, 3).reshape(-1, tile * tile)
+    raise ValueError(f"unknown tiling {tiling!r}")
+
+
+def tile_errors(got: torch.Tensor, ref: torch.Tensor, tiling: str, hkv: Optional[int] = None, tile: int = 128) -> dict:
+    """Error of ``got`` against the fp32 / fp64 ``ref``, tile by tile, so that an error confined to one head, one row block
+    or one GEMM tile is not averaged away by the rest of the tensor.
+
+    ``tiling``: ``"attn"`` ([B,S,H,D], one tile per (batch, head, 128 query rows)), ``"decode"`` ([B,Hq,D], one tile per
+    (batch, kv head); ``hkv`` = number of KV heads) or ``"2d"`` (a [T,N] output, one tile per 128 x 128 block).
+    Returns, over the tiles whose reference is not all zero, ``mean_rel`` = mean|err| / mean|ref| and ``max_rel`` =
+    max|err| / max|ref| (fp64 tensors, one value per tile), and ``empty_max`` = max|got| over the tiles whose reference is
+    all zero (they carry no relative error, so a value written there is reported as it is)."""
+    got, ref = got.double().cpu(), ref.double().cpu()
+    if got.shape != ref.shape:
+        raise ValueError(f"shapes differ: {tuple(got.shape)} vs {tuple(ref.shape)}")
+    err = _tiles((got - ref).abs(), tiling, hkv, tile)
+    mag = _tiles(ref.abs(), tiling, hkv, tile)
+    live = mag.amax(dim=1) > 0
+    dead = _tiles(got.abs(), tiling, hkv, tile)[~live]
+    return {
+        "mean_rel": err[live].sum(dim=1) / mag[live].sum(dim=1),
+        "max_rel": err[live].amax(dim=1) / mag[live].amax(dim=1),
+        "empty_max": float(dead.max()) if dead.numel() else 0.0,
+    }
 
 
 # --------------------------------------------------------------------------------------------------------------
