@@ -100,6 +100,24 @@ __device__ __forceinline__ int num_kv_tiles(const Params& p, int row0, int kv_le
   return static_cast<int>((visible + BLOCK_N - 1) / BLOCK_N);
 }
 
+// Zero rows [first, BLOCK_N) of a K/V tile in shared memory: the V rows at or past kv_len of the one tile per item that
+// straddles it. Those keys are masked (P = 0, or 2^-125 on the exp2_poly2 path), but 0 * NaN / Inf in P V is still NaN,
+// so padding that holds non-finite values (stale paged blocks, an uninitialised cache) would poison whole output rows.
+// Whole 128-byte rows can be zeroed as they are: the 128-byte swizzle permutes 16-byte chunks inside a row, never across
+// rows. Called by a whole warp; the proxy fence orders the stores before the tensor core reads the tile. Out of line: it
+// runs at most once per item, and inlined into the MMA issuer it added spills to the kernel.
+template <int BOXES>
+__device__ __noinline__ void zero_tile_rows(uint8_t* tile, int first, int lane) {
+  const int chunks = (BLOCK_N - first) * 8;  // 16-byte chunks per 64-column box
+#pragma unroll
+  for (int c = 0; c < BOXES; ++c) {
+    uint4* rows = reinterpret_cast<uint4*>(tile + c * 16384 + first * 128);
+    for (int i = lane; i < chunks; i += 32) rows[i] = make_uint4(0, 0, 0, 0);
+  }
+  fence_proxy_async_smem();
+  __syncwarp();
+}
+
 // One work item = one block index of the launch grid: a pair of 128-row query tiles of one (batch, head).
 struct Work {
   int head, batch, kv_head, q_row0, kv_len, n0, n1, n_max;
@@ -353,6 +371,8 @@ fa_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant_
           if (k_stage == NS) { k_stage = 0; k_phase ^= 1; }
           const bool has_next = (j + 1 < w.n_max);
           mbar_wait(&kv_full[v_stage], v_phase);
+          if (w.kv_len - j * BLOCK_N < BLOCK_N)  // V(j) straddles kv_len: its rows past the end must read as zeros
+            zero_tile_rows<C::BOXES>(smem + C::SMEM_KV_OFF + v_stage * C::TILE_BYTES, w.kv_len - j * BLOCK_N, lane);
           bool next_k_ready = false;
 #pragma unroll
           for (int t = 0; t < 2; ++t) {
@@ -867,6 +887,10 @@ fa_fwd_pair_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_cons
         const int j = s - 2;
         mbar_wait(&kv_full[stage], phase);
         if (j < n_mine) {
+          // V(j) straddles kv_len: this CTA zeroes its own copy of the multicast tile (the stage is refilled only once both
+          // CTAs have released it)
+          if (kv_len - j * BLOCK_N < BLOCK_N)
+            zero_tile_rows<C::BOXES>(smem + C::SMEM_KV_OFF + stage * C::TILE_BYTES, kv_len - j * BLOCK_N, lane);
           const int buf = j & 1;
           const uint32_t par = static_cast<uint32_t>((j >> 1) & 1);
           mbar_wait(&p_half[buf], par);        // (p_half[half][group])

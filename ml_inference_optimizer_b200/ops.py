@@ -89,7 +89,8 @@ def flash_attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, causal: bo
     """Attention forward. q ``[B,Sq,Hq,D]``, k/v ``[B,Sk,Hkv,D]`` (any batch/seq/head strides, D contiguous).
 
     Returns ``o [B,Sq,Hq,D]`` (same dtype as q) and, if ``return_lse``, ``lse [B,Hq,Sq]`` fp32 (natural log).
-    ``causal_offset`` = global position of query row 0 minus global position of key row 0.
+    ``causal_offset`` = global position of query row 0 minus global position of key row 0. Keys at or past
+    ``kv_lens[b]`` never affect the result, whatever they hold (NaN and Inf included).
     """
     if q.dim() != 4 or k.dim() != 4 or v.dim() != 4:
         raise ValueError(f"expected 4-D [B,S,H,D] tensors, got {tuple(q.shape)}, {tuple(k.shape)}, {tuple(v.shape)}")
@@ -162,7 +163,9 @@ def paged_prefill_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: tor
                             out: Optional[torch.Tensor] = None):
     """Short-q / chunked-prefill attention against the paged cache: q ``[B,Sq,Hq,D]`` are the LAST ``Sq`` tokens of every
     sequence (their K/V already appended), cache ``[num_blocks, L, block_size, Hkv, D]``, ``context_lens`` int32 ``[B]``
-    counts all keys. ``causal``: query i sees keys up to ``context_lens[b] - Sq + i``."""
+    counts all keys. ``causal``: query i sees keys up to ``context_lens[b] - Sq + i``. Cache slots at or past
+    ``context_lens[b]``, blocks the table does not name for the sequence and the other layers never affect the result,
+    whatever they hold (NaN and Inf included)."""
     dev = _require_cuda(q, k_cache, v_cache, block_tables, context_lens, out)
     if q.dim() != 4 or k_cache.dim() != 5 or v_cache.shape != k_cache.shape:
         raise ValueError("expected q [B,Sq,Hq,D] and caches [num_blocks, L, block_size, Hkv, D]")
@@ -227,6 +230,8 @@ def cast_out(o_acc: torch.Tensor, dtype: torch.dtype, out: Optional[torch.Tensor
         raise ValueError("o_acc must be a contiguous fp32 tensor")
     if out is None:
         out = torch.empty((B, Sq, Hq, D), dtype=dtype, device=dev)
+    elif tuple(out.shape) != (B, Sq, Hq, D) or out.dtype != dtype or out.stride(-1) != 1:
+        raise ValueError(f"out must be {dtype} of shape {(B, Sq, Hq, D)} with a contiguous last dimension")
     lib = _lib.load()
     with torch.cuda.device(dev):
         rc = lib.b200_cast_out(o_acc.data_ptr(), out.data_ptr(), B, Sq, Hq, D, strides3(out.stride()[:3]),
@@ -272,6 +277,8 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
         raise ValueError("cache dtype must match q")
     if context_lens.dtype != torch.int32 or not context_lens.is_contiguous() or context_lens.numel() != B:
         raise ValueError("context_lens must be a contiguous int32 [B] tensor")
+    if out is not None and (tuple(out.shape) != (B, Hq, D) or out.dtype != q.dtype or not out.is_contiguous()):
+        raise ValueError(f"out must be a contiguous {q.dtype} tensor of shape {(B, Hq, D)} (the kernels write it densely)")
     q = q.contiguous()
     paged = block_tables is not None
     if paged:
@@ -379,6 +386,19 @@ def activation_code(name) -> int:
         raise ValueError(f"unsupported activation {name!r}; supported: {sorted(k for k in _ACTIVATIONS if k)}") from None
 
 
+def _out_rows(out: torch.Tensor, lead: Tuple[int, ...], width: int, dtype: torch.dtype) -> torch.Tensor:
+    """``out`` seen as ``[rows, width]`` without a copy: the kernels write through its pointer and one row stride, so an
+    ``out`` they cannot address that way is refused rather than written into a temporary the caller never sees."""
+    if tuple(out.shape) != (*lead, width) or out.dtype != dtype:
+        raise ValueError(f"out must be {dtype} of shape {(*lead, width)}, got {out.dtype} {tuple(out.shape)}")
+    if out.stride(-1) != 1:
+        raise ValueError("out must have a contiguous last dimension")
+    try:
+        return out.view(-1, width)
+    except RuntimeError:
+        raise ValueError(f"out (strides {out.stride()}) cannot be addressed as rows of one stride") from None
+
+
 def _as_rows(x: torch.Tensor) -> Tuple[torch.Tensor, Tuple[int, ...]]:
     lead = tuple(x.shape[:-1])
     x2 = x.reshape(-1, x.shape[-1])
@@ -409,7 +429,7 @@ def linear_act(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tenso
             raise ValueError("SwiGLU needs gate_weight")
         gate_weight = gate_weight.contiguous()
         gate_bias = None if gate_bias is None else gate_bias.contiguous()
-    y = out.reshape(-1, N) if out is not None else torch.empty((T, N), dtype=x.dtype, device=dev)
+    y = _out_rows(out, lead, N, x.dtype) if out is not None else torch.empty((T, N), dtype=x.dtype, device=dev)
     lib = _lib.load()
     with torch.cuda.device(dev):
         ws_bytes = lib.b200_linear_act_workspace_bytes(T, K, N, act)
@@ -418,7 +438,7 @@ def linear_act(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tenso
                                  _ptr(gate_weight), _ptr(gate_bias), y.data_ptr(), y.stride(0) if T > 1 else N, T, K, N,
                                  act, _ptr(ws), ws_bytes, dt, _stream_ptr(dev))
     check("b200_linear_act", rc)
-    return y.reshape(*lead, N)
+    return out if out is not None else y.reshape(*lead, N)
 
 
 def fused_mlp(x: torch.Tensor, w_up: torch.Tensor, b_up: Optional[torch.Tensor], w_down: torch.Tensor,
@@ -453,7 +473,7 @@ def fused_mlp(x: torch.Tensor, w_up: torch.Tensor, b_up: Optional[torch.Tensor],
     b_up = None if b_up is None else b_up.contiguous()
     b_down = None if b_down is None else b_down.contiguous()
     b_gate = None if b_gate is None else b_gate.contiguous()
-    y = out.reshape(-1, h_out) if out is not None else torch.empty((T, h_out), dtype=x.dtype, device=dev)
+    y = _out_rows(out, lead, h_out, x.dtype) if out is not None else torch.empty((T, h_out), dtype=x.dtype, device=dev)
     lib = _lib.load()
     with torch.cuda.device(dev):
         ws_bytes = lib.b200_fused_mlp_workspace_bytes(T, h, i)
@@ -473,13 +493,13 @@ def fused_mlp(x: torch.Tensor, w_up: torch.Tensor, b_up: Optional[torch.Tensor],
                                      _stream_ptr(dev))
             check("b200_linear_act", rc)
             e2.record(stream)
-            return y.reshape(*lead, h_out)
+            return out if out is not None else y.reshape(*lead, h_out)
         rc = lib.b200_fused_mlp(x2.data_ptr(), x2.stride(0) if T > 1 else h, w_up.data_ptr(), _ptr(b_up), _ptr(w_gate),
                                 _ptr(b_gate), w_down.data_ptr(), _ptr(b_down), y.data_ptr(),
                                 y.stride(0) if T > 1 else h_out, T, h, i, h_out, act, _ptr(ws), ws_bytes, dt,
                                 _stream_ptr(dev))
     check("b200_fused_mlp", rc)
-    return y.reshape(*lead, h_out)
+    return out if out is not None else y.reshape(*lead, h_out)
 
 
 def layernorm(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor] = None, eps: float = 1e-5,
@@ -501,14 +521,14 @@ def layernorm(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor
     weight = weight.contiguous()
     bias = None if bias is None else bias.contiguous()
     rows = x2.shape[0]
-    y = out.reshape(-1, cols) if out is not None else torch.empty((rows, cols), dtype=x.dtype, device=dev)
+    y = _out_rows(out, lead, cols, x.dtype) if out is not None else torch.empty((rows, cols), dtype=x.dtype, device=dev)
     ld = lambda t: t.stride(0) if t.shape[0] > 1 else cols
     lib = _lib.load()
     with torch.cuda.device(dev):
         rc = lib.b200_layernorm(x2.data_ptr(), _ptr(r2), weight.data_ptr(), _ptr(bias), y.data_ptr(), rows, cols, ld(x2),
                                 ld(r2) if r2 is not None else 0, ld(y), float(eps), float(residual_alpha), dt, _stream_ptr(dev))
     check("b200_layernorm", rc)
-    return y.reshape(*lead, cols)
+    return out if out is not None else y.reshape(*lead, cols)
 
 
 def set_sm_limit(max_ctas: int) -> None:
