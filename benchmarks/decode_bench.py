@@ -26,7 +26,10 @@ def main():
     ap.add_argument("--prompt", type=int, default=64)
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--cpu-tokens", type=int, default=24)
+    ap.add_argument("--kv-cache-dtype", choices=["bf16", "fp8"], default="bf16",
+                    help="paged KV cache of the b200 legs: bf16, or fp8 (e4m3, scales 1.0)")
     args = ap.parse_args()
+    kv_dtype = torch.float8_e4m3fn if args.kv_cache_dtype == "fp8" else None
     from transformers import GPT2Config, GPT2LMHeadModel
 
     from ml_inference_optimizer_b200.baseline.inference import generate_paged
@@ -39,7 +42,7 @@ def main():
 
     def emit(leg, tokens, seconds, **extra):
         print(json.dumps({"bench": "gpt2_small_generate", "leg": leg, "batch": args.batch, "prompt": args.prompt,
-                          "new_tokens": tokens, "seconds": seconds, "tokens_per_s": args.batch * tokens / seconds, **extra}),
+                          "kv_cache_dtype": args.kv_cache_dtype, "new_tokens": tokens, "seconds": seconds, "tokens_per_s": args.batch * tokens / seconds, **extra}),
               flush=True)
 
     if args.cpu_tokens > 0:
@@ -69,10 +72,11 @@ def main():
     emit("gpu_hf_generate_bf16", args.new_tokens, sec)
     import copy
     ours = Optimizer(copy.deepcopy(hf)).optimize(use_flash_attention=True, use_fused_mlp=True)
-    out_e, sec = timed(lambda: generate_paged(ours, gids, args.new_tokens))
+    out_e, sec = timed(lambda: generate_paged(ours, gids, args.new_tokens, kv_cache_dtype=kv_dtype))
     emit("b200_paged_eager_launches", args.new_tokens, sec, agree_with_hf=float((out_e == ref).float().mean()))
     try:
-        out_g, sec = timed(lambda: generate_paged(ours, gids, args.new_tokens, use_cuda_graph=True))
+        out_g, sec = timed(lambda: generate_paged(ours, gids, args.new_tokens, use_cuda_graph=True,
+                                                       kv_cache_dtype=kv_dtype))
         from ml_inference_optimizer_b200.baseline.inference import LAST_DECODE_STATS as st
         emit("b200_paged_cuda_graph", args.new_tokens, sec, agree_with_eager=float((out_g == out_e).float().mean()),
              capture_seconds=st.get("capture_s"), replay_steps=st.get("replay_steps"), replay_ms=st.get("replay_ms"),

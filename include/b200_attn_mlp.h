@@ -166,6 +166,29 @@ int b200_kv_append(const void* key, const void* value, void* k_cache, void* v_ca
                    const int32_t* block_table, int max_blocks_per_seq, int block_size, int num_layers,
                    int layer_idx, int dtype, void* stream);
 
+/* ---- FP8 (e4m3) paged KV cache: quantizing append and decode ------------------------------------------------
+ * Format (the same for every writer and reader): element torch.float8_e4m3fn, one fp32 k_scale and one v_scale per
+ * layer (> 0 and finite). Stored byte = cvt.rn.satfinite.e4m3(x / scale) with a correctly rounded fp32 division:
+ * |x / scale| past 448 and +-inf saturate to +-448, NaN stays NaN. Value read = byte * scale. Paged layout only:
+ * [num_blocks, L, block_size, Hkv, D] bytes, D in {64, 128}.
+ *
+ * b200_kv_append_fp8: key, value [B, n_tokens, Hkv, D] contiguous, bf16 or fp16 (dtype). Row i of sequence b goes to
+ *   position context_lens[b] - n_tokens + i: n_tokens = 1 is the decode append, n_tokens = S the prompt of prefill.
+ *   Positions below 0 or >= max_blocks_per_seq * block_size are dropped, as in b200_kv_append.
+ * b200_fa_decode_fp8: the contract of b200_fa_decode for the paged layout, over an FP8 cache; q / o bf16 or fp16, lse
+ *   optional, same split rule (b200_fa_decode_num_splits) and workspace size (b200_fa_decode_workspace_bytes).
+ *   k_scale is folded into softmax_scale, v_scale multiplies each output row. B200_KV_CONTIGUOUS returns
+ *   B200_ERR_UNSUPPORTED. Cache bytes at or past context_lens[b] are never read.                                */
+int b200_kv_append_fp8(const void* key, const void* value, void* k_cache, void* v_cache, int B, int n_tokens, int Hkv,
+                       int D, const int32_t* context_lens, const int32_t* block_table, int max_blocks_per_seq,
+                       int block_size, int num_layers, int layer_idx, float k_scale, float v_scale, int dtype,
+                       void* stream);
+int b200_fa_decode_fp8(const void* q, const void* k_cache, const void* v_cache, void* o, float* lse, int B, int Hq,
+                       int Hkv, int D, const int32_t* context_lens, int max_context_len, float softmax_scale, int layout,
+                       const int32_t* block_table, int max_blocks_per_seq, int block_size, int num_layers,
+                       int layer_idx, int num_splits, void* workspace, int64_t workspace_bytes, float k_scale,
+                       float v_scale, int dtype, void* stream);
+
 /* ---- K3: FusedMLP ---------------------------------------------------------------------------------------
  * Replaces triton_fused_mlp (kernels/triton/mlp_kernels.py:648-756) and FusedMLP*._forward_*
  *   (kernels/mlp/fused_mlp.py:59-72, :159-178, :223-237, :262-275):

@@ -48,6 +48,11 @@ SIGNATURES = {
                                c_void_p, c_int64, c_int, c_void_p]),
     "b200_kv_append": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int64,
                                c_int64, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "b200_fa_decode_fp8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
+                                   c_int, c_float, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int64,
+                                   c_float, c_float, c_int, c_void_p]),
+    "b200_kv_append_fp8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
+                                   c_int, c_int, c_int, c_int, c_float, c_float, c_int, c_void_p]),
     "b200_fused_mlp_workspace_bytes": (c_int64, [c_int64, c_int, c_int]),
     "b200_fused_mlp": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                c_int64, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_int64, c_int, c_void_p]),

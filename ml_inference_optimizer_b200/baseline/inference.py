@@ -93,15 +93,37 @@ class SequenceMetadata:
         return len(self.block_table)
 
 
+def _per_layer_scales(name: str, scale: Union[float, Sequence[float]], num_layers: int) -> List[float]:
+    vals = [float(scale)] * num_layers if isinstance(scale, (int, float)) else [float(x) for x in scale]
+    if len(vals) != num_layers:
+        raise ValueError(f"{name} has {len(vals)} values for {num_layers} layers")
+    if not all(math.isfinite(x) and x > 0 for x in vals):
+        raise ValueError(f"{name} values must be positive and finite, got {vals}")
+    return vals
+
+
 class PagedKVCache:
-    """reference :1150-1302."""
+    """reference :1150-1302.
+
+    ``dtype=torch.float8_e4m3fn`` stores K and V as e4m3 bytes: half the memory of a 16-bit cache, read by the FP8 decode
+    kernels. ``k_scale`` / ``v_scale`` (a float, or one value per layer) are what a stored byte is multiplied by when it is
+    read (K is stored as e4m3(K / k_scale)); a 16-bit cache takes only 1.0."""
 
     def __init__(self, num_blocks: int, block_size: int, num_layers: int, num_heads: int, head_dim: int,
-                 dtype: torch.dtype = torch.float16, device: str = "cuda"):
+                 dtype: torch.dtype = torch.float16, device: str = "cuda", k_scale: Union[float, Sequence[float]] = 1.0,
+                 v_scale: Union[float, Sequence[float]] = 1.0):
+        self.k_scales = _per_layer_scales("k_scale", k_scale, num_layers)
+        self.v_scales = _per_layer_scales("v_scale", v_scale, num_layers)
+        if dtype != torch.float8_e4m3fn and any(x != 1.0 for x in self.k_scales + self.v_scales):
+            raise ValueError("k_scale / v_scale apply to an FP8 (torch.float8_e4m3fn) cache only")
         self.block_manager = BlockManager(num_blocks, block_size, num_layers, num_heads, head_dim, dtype, device)
         self.block_size, self.num_layers, self.num_heads, self.head_dim = block_size, num_layers, num_heads, head_dim
         self.dtype, self.device = dtype, device
         self.sequences: Dict[int, SequenceMetadata] = {}
+
+    def layer_scales(self, layer_idx: int) -> Tuple[float, float]:
+        """``(k_scale, v_scale)`` of one layer: a stored K / V byte is worth ``byte * scale``."""
+        return self.k_scales[layer_idx], self.v_scales[layer_idx]
 
     def _ensure_sequence_exists(self, seq_id: int):
         if seq_id not in self.sequences:
@@ -176,9 +198,17 @@ class PagedKVCache:
         return bt.to(self.device), lens.to(self.device)
 
     def write_prefill(self, layer_idx: int, seq_ids: List[int], k: torch.Tensor, v: torch.Tensor) -> None:
-        """Scatter the prompt's K,V ``[B,S,Hkv,D]`` into the blocks (prefill; the per-token path is ``b200_kv_append``)."""
+        """Scatter the prompt's K,V ``[B,S,Hkv,D]`` into the blocks (prefill; the per-token path is ``b200_kv_append``).
+        An FP8 cache is written by ``b200_kv_append_fp8`` with all S rows at once, so prefill and decode quantize alike."""
         kc, vc = self.get_physical_caches()
         B, S = k.shape[:2]
+        if self.dtype == torch.float8_e4m3fn:
+            from .. import ops
+            bt, _ = self.device_tables(seq_ids)
+            lens = torch.full((B,), S, dtype=torch.int32, device=bt.device)
+            ks, vs = self.layer_scales(layer_idx)
+            ops.kv_append(k, v, kc, vc, lens, bt, layer_idx, k_scale=ks, v_scale=vs)
+            return
         pos = torch.arange(S)
         for b, sid in enumerate(seq_ids):
             table = torch.tensor(self.get_block_table(sid), dtype=torch.long)
@@ -394,8 +424,10 @@ class TransformerInferenceRunner(InferenceRunner):
 
     def __init__(self, model: nn.Module, device: str, precision: str = "fp16", is_encoder_decoder: bool = False,
                  use_kv_cache: bool = True, use_cuda_graph: bool = False, use_paged_attention: bool = True,
-                 kv_cache_num_gpu_blocks: Optional[int] = None, kv_cache_block_size: int = 16):
+                 kv_cache_num_gpu_blocks: Optional[int] = None, kv_cache_block_size: int = 16,
+                 kv_cache_dtype: Optional[torch.dtype] = None):
         super().__init__(model, device, precision)
+        self.kv_cache_dtype = kv_cache_dtype   # None: the model's dtype; torch.float8_e4m3fn: the FP8 paged cache
         cuda = str(device).startswith("cuda")
         self.is_encoder_decoder = is_encoder_decoder
         self.use_kv_cache = use_kv_cache and cuda
@@ -441,7 +473,8 @@ class TransformerInferenceRunner(InferenceRunner):
         total = torch.cuda.get_device_properties(dev).total_memory
         weights = sum(p.numel() for p in self.model.parameters()) * 2
         avail = total - torch.cuda.memory_allocated(dev) - 4 * weights - 0.10 * total
-        per_block = 2 * self.num_layers * self.kv_cache_block_size * self.num_heads * self.head_dim * 2
+        elem = 1 if self.kv_cache_dtype == torch.float8_e4m3fn else 2
+        per_block = 2 * self.num_layers * self.kv_cache_block_size * self.num_heads * self.head_dim * elem
         if per_block == 0 or avail <= 0:
             return 0
         return int(min(avail, 0.8 * total) // per_block)
@@ -453,7 +486,7 @@ class TransformerInferenceRunner(InferenceRunner):
             logging.warning("Model parameters not detected. Cannot initialize KV cache.")
             self.use_kv_cache = False
             return
-        dtype = next(self.model.parameters()).dtype
+        dtype = self.kv_cache_dtype or next(self.model.parameters()).dtype
         if self.use_paged_attention:
             if self.kv_cache_num_gpu_blocks is None:
                 self.kv_cache_num_gpu_blocks = self._calculate_num_gpu_blocks()
@@ -616,22 +649,30 @@ def _adapters(model: nn.Module) -> List[_fa._HFAttentionAdapter]:
 
 
 def generate_paged(model: nn.Module, input_ids: torch.Tensor, max_new_tokens: int, cache: Optional[PagedKVCache] = None,
-                   block_size: int = 16, use_cuda_graph: bool = False) -> torch.Tensor:
+                   block_size: int = 16, use_cuda_graph: bool = False,
+                   kv_cache_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """Greedy generation with the paged KV cache: prefill runs K1 and scatters the prompt's K,V into blocks; every decode
     step appends the new token's K,V (``b200_kv_append``) and attends through the block tables (K2). Returns
     ``[B, S + max_new_tokens]`` token ids.
 
     ``use_cuda_graph=True`` captures one decode step (all layers: projections, KV append, K2, MLP, LM head, argmax) in a
     CUDA graph and replays it: block tables are reserved up front, lengths / positions / the token are advanced on the
-    device, so a step has no host work besides the replay (the loop is launch-bound otherwise)."""
+    device, so a step has no host work besides the replay (the loop is launch-bound otherwise).
+
+    ``kv_cache_dtype=torch.float8_e4m3fn`` allocates an FP8 cache (scales 1.0) when no ``cache`` is passed."""
     adapters = _adapters(model)
     first = adapters[0].inner
     B, S = input_ids.shape
     dev = input_ids.device
+    compute = first.flash_attention._compute_dtype(next(model.parameters()).dtype)
+    if kv_cache_dtype not in (None, compute, torch.float8_e4m3fn):
+        raise ValueError(f"kv_cache_dtype must be None, {compute} or torch.float8_e4m3fn, got {kv_cache_dtype}")
     if cache is None:
         blocks = B * math.ceil((S + max_new_tokens) / block_size) + 1
-        dtype = first.flash_attention._compute_dtype(next(model.parameters()).dtype)
-        cache = PagedKVCache(blocks, block_size, len(adapters), first.num_kv_heads, first.head_dim, dtype=dtype, device=str(dev))
+        cache = PagedKVCache(blocks, block_size, len(adapters), first.num_kv_heads, first.head_dim,
+                             dtype=kv_cache_dtype or compute, device=str(dev))
+    elif kv_cache_dtype is not None and cache.dtype != kv_cache_dtype:
+        raise ValueError(f"kv_cache_dtype {kv_cache_dtype} differs from the dtype of the cache passed ({cache.dtype})")
     seq_ids = list(range(B))
     for sid in seq_ids:
         cache.allocate_blocks_for_sequence(sid, S)

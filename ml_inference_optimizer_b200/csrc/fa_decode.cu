@@ -742,6 +742,518 @@ int dispatch_group(int G, const Params& p, bool paged, cudaStream_t stream) {
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// FP8 (e4m3) paged KV cache. One format for every writer and reader:
+//   stored byte = cvt.rn.satfinite.e4m3(x / scale)   x in fp32, correctly rounded division (__fdiv_rn); |x / scale| past
+//                                                     448 and +-inf saturate to +-448, NaN stays NaN
+//   value read  = byte * scale                        one fp32 k_scale and one v_scale per layer
+// The readers never multiply per element: k_scale is folded into the softmax scale on the host, v_scale multiplies each
+// output row once before its store. Half the bytes of a 16-bit cache: decode streams half as much from HBM, and the same
+// memory holds twice the tokens.
+// uint4 values are built by aggregate initialisation, not make_uint4: more call sites of that static inline header
+// function change how NVVM inlines it into decode_gqa_mma_kernel, and the 16-bit kernels must compile as before.
+// ---------------------------------------------------------------------------------------------------------------
+namespace fp8 {
+
+// two fp32 -> two e4m3 bytes (lo in bits 0-7, hi in bits 8-15)
+__device__ __forceinline__ uint32_t quant2(float lo, float hi, float scale) {
+  uint16_t r;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(__fdiv_rn(hi, scale)), "f"(__fdiv_rn(lo, scale)));
+  return r;
+}
+// four 16-bit values (two packed words) -> four bytes
+template <typename T>
+__device__ __forceinline__ uint32_t quant4(uint32_t a, uint32_t b, float scale) {
+  const float2 x = Pack2<T>::unpack(a), y = Pack2<T>::unpack(b);
+  return quant2(x.x, x.y, scale) | (quant2(y.x, y.y, scale) << 16);
+}
+// the two e4m3 bytes in bits 0-15 of v -> f16x2 (byte 0 in the low half); exact: every e4m3 value is an f16 value
+__device__ __forceinline__ uint32_t widen2(uint32_t v) {
+  uint32_t r;
+  asm("cvt.rn.f16x2.e4m3x2 %0, %1;" : "=r"(r) : "h"(static_cast<uint16_t>(v)));
+  return r;
+}
+__device__ __forceinline__ float2 half2_to_float2(uint32_t h) { return Pack2<__half>::unpack(h); }
+// ld_stream predicated on `valid` (zeros otherwise), without a branch: keeps the staged tiles in registers
+__device__ __forceinline__ uint4 ld_stream_if(const void* p, bool valid) {
+  uint4 r;
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %5, 0;\n\t"
+               "mov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
+               "@q ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];\n\t}"
+               : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w)
+               : "l"(p), "r"(static_cast<int>(valid)));
+  return r;
+}
+__device__ __forceinline__ uint2 ld_stream8_if(const void* p, bool valid) {
+  uint2 r;
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %3, 0;\n\tmov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\t"
+               "@q ld.global.nc.L1::no_allocate.v2.u32 {%0, %1}, [%2];\n\t}"
+               : "=r"(r.x), "=r"(r.y)
+               : "l"(p), "r"(static_cast<int>(valid)));
+  return r;
+}
+
+// Quantizing append: the n_tokens newest K,V rows of every sequence ([B, n_tokens, Hkv, D], 16-bit) go to positions
+// [context_lens[b] - n_tokens, context_lens[b]). n_tokens = 1 is the decode append, n_tokens = S the prompt scatter of
+// prefill, so both quantize by the same rule. A position past the cache is dropped, as in kv_append_kernel. Each thread
+// turns 16 values (two 16-byte loads) into one 16-byte store.
+template <typename T>
+__global__ void kv_append_kernel(const T* __restrict__ key, const T* __restrict__ value, uint8_t* __restrict__ k_cache,
+                                 uint8_t* __restrict__ v_cache, const int32_t* __restrict__ context_lens, int n_tokens,
+                                 int row_elems, const int32_t* __restrict__ block_table, int max_blocks_per_seq,
+                                 int block_size, int num_layers, int layer_idx, float k_scale, float v_scale) {
+  const int i = blockIdx.x, b = blockIdx.y;
+  const int pos = context_lens[b] - n_tokens + i;
+  if (pos < 0 || pos >= max_blocks_per_seq * block_size) return;
+  const int bi = pos / block_size;
+  const int in_blk = pos - bi * block_size;
+  const int blk = block_table[static_cast<int64_t>(b) * max_blocks_per_seq + bi];
+  const int64_t dst = ((static_cast<int64_t>(blk) * num_layers + layer_idx) * block_size + in_blk) * row_elems;
+  const int64_t src = (static_cast<int64_t>(b) * n_tokens + i) * row_elems;
+  const uint4* ks = reinterpret_cast<const uint4*>(key + src);
+  const uint4* vs = reinterpret_cast<const uint4*>(value + src);
+  uint4* kd = reinterpret_cast<uint4*>(k_cache + dst);
+  uint4* vd = reinterpret_cast<uint4*>(v_cache + dst);
+  for (int c = threadIdx.x; c < row_elems / 16; c += blockDim.x) {
+    const uint4 k0 = ks[2 * c], k1 = ks[2 * c + 1], v0 = vs[2 * c], v1 = vs[2 * c + 1];
+    kd[c] = uint4{quant4<T>(k0.x, k0.y, k_scale), quant4<T>(k0.z, k0.w, k_scale), quant4<T>(k1.x, k1.y, k_scale),
+                       quant4<T>(k1.z, k1.w, k_scale)};
+    vd[c] = uint4{quant4<T>(v0.x, v0.y, v_scale), quant4<T>(v0.z, v0.w, v_scale), quant4<T>(v1.x, v1.y, v_scale),
+                       quant4<T>(v1.z, v1.w, v_scale)};
+  }
+}
+
+// 16 e4m3 bytes -> 16 floats
+__device__ __forceinline__ void widen16(const uint4 r, float (&f)[16]) {
+  const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 a = half2_to_float2(widen2(w[j])), c = half2_to_float2(widen2(w[j] >> 16));
+    f[4 * j] = a.x; f[4 * j + 1] = a.y; f[4 * j + 2] = c.x; f[4 * j + 3] = c.y;
+  }
+}
+
+// G = 1, 2 on CUDA cores, the loop of decode_kernel over e4m3 rows: a 16-byte load carries 16 values, so D/16 lanes
+// cover a row and a warp-wide load covers twice the rows of the 16-bit kernel. p.scale_log2 includes k_scale.
+template <int D, int G, typename T>
+__global__ void __launch_bounds__(NUM_THREADS, 2)
+decode_kernel(const Params p, const float v_scale) {
+  constexpr int NLOAD = 8 / G;        // 16-byte loads in flight per lane for K (and again for V); G = 2 needs the registers
+  constexpr int LPR = D / 16;         // lanes per KV row
+  constexpr int RPW = 32 / LPR;       // rows per warp-wide load
+  constexpr int TILE = NLOAD * RPW;   // keys per warp iteration
+
+  const int split = blockIdx.x, kvh = blockIdx.y, b = blockIdx.z;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int sub = lane % LPR;         // which 16-element slice of the row
+  const int rsel = lane / LPR;        // which row of the warp-wide load
+
+  const int ctx = max(0, min(p.context_lens[b], p.capacity));
+  int chunk = (ctx + p.splits - 1) / p.splits;
+  chunk = ((chunk + TILE - 1) / TILE) * TILE;
+  const int k_begin = min(split * chunk, ctx);
+  const int k_end = min(k_begin + chunk, ctx);
+
+  float qf[G][16];
+#pragma unroll
+  for (int g = 0; g < G; ++g) {
+    const T* qp = reinterpret_cast<const T*>(p.q) + (static_cast<int64_t>(b) * p.Hq + kvh * G + g) * D + sub * 16;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const uint4 raw = *reinterpret_cast<const uint4*>(qp + 8 * h);
+      const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 f = Pack2<T>::unpack(w[j]);
+        qf[g][8 * h + 2 * j] = f.x * p.scale_log2;
+        qf[g][8 * h + 2 * j + 1] = f.y * p.scale_log2;
+      }
+    }
+  }
+  float m_run[G], l_run[G], acc[G][16];
+#pragma unroll
+  for (int g = 0; g < G; ++g) {
+    m_run[g] = -INFINITY;
+    l_run[g] = 0.f;
+#pragma unroll
+    for (int e = 0; e < 16; ++e) acc[g][e] = 0.f;
+  }
+
+  const uint8_t* kc = reinterpret_cast<const uint8_t*>(p.k_cache);
+  const uint8_t* vc = reinterpret_cast<const uint8_t*>(p.v_cache);
+  const int32_t* bt = p.block_table + static_cast<int64_t>(b) * p.max_blocks_per_seq;
+  const bool bs_pow2 = (p.block_size & (p.block_size - 1)) == 0;
+  const int bs_shift = bs_pow2 ? (31 - __clz(p.block_size)) : 0;
+
+  for (int t0 = k_begin + warp * TILE; t0 < k_end; t0 += NUM_WARPS * TILE) {
+    uint4 kraw[NLOAD], vraw[NLOAD];
+    bool valid[NLOAD];
+#pragma unroll
+    for (int i = 0; i < NLOAD; ++i) {
+      const int key = t0 + i * RPW + rsel;
+      valid[i] = key < k_end;
+      if (valid[i]) {   // bytes of keys at or past the end are never loaded
+        const int bi = bs_pow2 ? (key >> bs_shift) : (key / p.block_size);
+        const int in_blk = bs_pow2 ? (key & (p.block_size - 1)) : (key - bi * p.block_size);
+        const int64_t off = ((static_cast<int64_t>(bt[bi]) * p.num_layers + p.layer_idx) * p.block_size + in_blk) *
+                                (static_cast<int64_t>(p.Hkv) * D) + kvh * D + sub * 16;
+        kraw[i] = ld_stream(kc + off);
+        vraw[i] = ld_stream(vc + off);
+      } else {
+        kraw[i] = uint4{0, 0, 0, 0};
+        vraw[i] = uint4{0, 0, 0, 0};
+      }
+    }
+    float s[G][NLOAD];
+#pragma unroll
+    for (int i = 0; i < NLOAD; ++i) {
+      float kf[16];
+      widen16(kraw[i], kf);
+#pragma unroll
+      for (int g = 0; g < G; ++g) {
+        float d = 0.f;
+#pragma unroll
+        for (int e = 0; e < 16; ++e) d = fmaf(qf[g][e], kf[e], d);
+#pragma unroll
+        for (int x = LPR / 2; x >= 1; x >>= 1) d += __shfl_xor_sync(0xffffffffu, d, x);
+        s[g][i] = valid[i] ? d : -INFINITY;
+      }
+    }
+    float pr[G][NLOAD];
+#pragma unroll
+    for (int g = 0; g < G; ++g) {
+      float tmax = s[g][0];
+#pragma unroll
+      for (int i = 1; i < NLOAD; ++i) tmax = fmaxf(tmax, s[g][i]);
+#pragma unroll
+      for (int x = LPR; x < 32; x <<= 1) tmax = fmaxf(tmax, __shfl_xor_sync(0xffffffffu, tmax, x));
+      const float m_new = fmaxf(m_run[g], tmax);
+      const float m_safe = (m_new == -INFINITY) ? 0.f : m_new;
+      const float corr = fast_exp2(m_run[g] - m_safe);
+      m_run[g] = m_new;
+      l_run[g] *= corr;
+#pragma unroll
+      for (int e = 0; e < 16; ++e) acc[g][e] *= corr;
+#pragma unroll
+      for (int i = 0; i < NLOAD; ++i) {
+        pr[g][i] = fast_exp2(s[g][i] - m_safe);
+        l_run[g] += pr[g][i];
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < NLOAD; ++i) {
+      float vf[16];
+      widen16(vraw[i], vf);
+#pragma unroll
+      for (int g = 0; g < G; ++g) {
+#pragma unroll
+        for (int e = 0; e < 16; ++e) acc[g][e] = fmaf(pr[g][i], vf[e], acc[g][e]);
+      }
+    }
+  }
+
+#pragma unroll
+  for (int g = 0; g < G; ++g) {
+#pragma unroll
+    for (int x = LPR; x < 32; x <<= 1) {
+      l_run[g] += __shfl_xor_sync(0xffffffffu, l_run[g], x);
+#pragma unroll
+      for (int e = 0; e < 16; ++e) acc[g][e] += __shfl_xor_sync(0xffffffffu, acc[g][e], x);
+    }
+  }
+  __shared__ float sm_m[NUM_WARPS][G];
+  __shared__ float sm_l[NUM_WARPS][G];
+  __shared__ float sm_acc[NUM_WARPS][G][D];
+  if (rsel == 0) {
+#pragma unroll
+    for (int g = 0; g < G; ++g) {
+#pragma unroll
+      for (int e = 0; e < 16; ++e) sm_acc[warp][g][sub * 16 + e] = acc[g][e];
+      if (sub == 0) {
+        sm_m[warp][g] = m_run[g];
+        sm_l[warp][g] = l_run[g];
+      }
+    }
+  }
+  __syncthreads();
+  for (int idx = threadIdx.x; idx < G * D; idx += NUM_THREADS) {
+    const int g = idx / D;
+    const int d = idx - g * D;
+    float m = -INFINITY;
+#pragma unroll
+    for (int w = 0; w < NUM_WARPS; ++w) m = fmaxf(m, sm_m[w][g]);
+    const float m_safe = (m == -INFINITY) ? 0.f : m;
+    float l = 0.f, o = 0.f;
+#pragma unroll
+    for (int w = 0; w < NUM_WARPS; ++w) {
+      const float c = fast_exp2(sm_m[w][g] - m_safe);
+      l = fmaf(sm_l[w][g], c, l);
+      o = fmaf(sm_acc[w][g][d], c, o);
+    }
+    const float out = l > 0.f ? o / l * v_scale : 0.f;
+    const float lse = l > 0.f ? (m + log2f(l)) * kLn2 : -INFINITY;
+    const int h = kvh * G + g;
+    if (p.splits == 1) {
+      T* op = reinterpret_cast<T*>(p.o) + (static_cast<int64_t>(b) * p.Hq + h) * D + d;
+      if constexpr (Pack2<T>::kIsBf16) *op = __float2bfloat16_rn(out);
+      else *op = __float2half_rn(out);
+      if (d == 0 && p.lse != nullptr) p.lse[static_cast<int64_t>(b) * p.Hq + h] = lse;
+    } else {
+      const int64_t row = (static_cast<int64_t>(b) * p.Hq + h) * p.splits + split;
+      p.part_o[row * D + d] = out;
+      if (d == 0) p.part_lse[row] = lse;
+    }
+  }
+}
+
+// G = 3..16 on mma.sync m16n8k16, the register-staged schedule of decode_gqa_mma_kernel over e4m3 rows.
+//   Q K^T : lane (g,t) loads K[key g][64m + 16t .. +16): one 16-byte load, widened to eight f16x2 words, feeds four
+//           k-steps (word pair j of the load is k-step j; the Q fragments carry the same permutation of the contraction
+//           index). A warp iteration covers 32 keys, four n-tiles of 8, so a tile is as many bytes as the 16-bit kernel's.
+//   P V   : lane (g,t) loads the D/8 bytes V[key][D/8 * g .. +D/8) of keys {2t, 2t+1, 2t+8, 2t+9} of each 16-key k-step;
+//           PRMT pairs byte j of two keys and one cvt widens the pair into a B fragment. Output column c of n-tile j is
+//           dim D/8 * c + j (undone at the final store).
+// The MMA runs in f16 for both q types. ptxas has no e4m3 -> bf16x2 conversion on sm_100a; an exact widening by bit
+// operations (shift the 7 magnitude bits into bf16 position, multiply by 2^120) costs four instructions per pair instead
+// of one, on a kernel whose issue slots already carry the MMAs, the widening and the softmax of twice the keys per byte.
+// A bf16 q is converted to f16 once per CTA instead: exact for |q| in [2^-14, 65504] (bf16 has 8 significant bits, f16
+// has 11), which covers the projected queries of a model by orders of magnitude; P in f16 rounds finer than bf16 would.
+template <int D, typename T>
+__global__ void __launch_bounds__(GQA_WARPS * 32, GqaMinCtas<D>::value)
+decode_gqa_mma_kernel(const Params p, const int G, const float v_scale) {
+  constexpr int TILE = 32;       // keys per warp iteration
+  constexpr int MB = D / 64;     // 64-dim blocks of the head dimension (one 16-byte K load per lane, four k-steps)
+  constexpr int VW = D / 8;      // V bytes a lane loads per key (= n-tiles of the P V product)
+  constexpr int VWORDS = VW / 4;
+
+  const int split = blockIdx.x, kvh = blockIdx.y, b = blockIdx.z;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = lane >> 2, t = lane & 3;
+
+  const int ctx = max(0, min(p.context_lens[b], p.capacity));
+  int chunk = (ctx + p.splits - 1) / p.splits;
+  chunk = ((chunk + TILE - 1) / TILE) * TILE;
+  const int k_begin = min(split * chunk, ctx);
+  const int k_end = min(k_begin + chunk, ctx);
+
+  // Q fragments (f16) for rows g and g+8 (zero rows beyond the group): word i of block m = dims 64m + 16t + 2i, +1
+  uint32_t qa[MB][8], qb[MB][8];
+  {
+    const T* qbase = reinterpret_cast<const T*>(p.q) + (static_cast<int64_t>(b) * p.Hq + kvh * G) * D;
+#pragma unroll
+    for (int m = 0; m < MB; ++m) {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        uint4 ra = uint4{0, 0, 0, 0}, rb = uint4{0, 0, 0, 0};
+        if (g < G) ra = *reinterpret_cast<const uint4*>(qbase + static_cast<int64_t>(g) * D + 64 * m + 16 * t + 8 * h);
+        if (g + 8 < G) rb = *reinterpret_cast<const uint4*>(qbase + static_cast<int64_t>(g + 8) * D + 64 * m + 16 * t + 8 * h);
+        const uint32_t wa[4] = {ra.x, ra.y, ra.z, ra.w}, wb[4] = {rb.x, rb.y, rb.z, rb.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          if constexpr (Pack2<T>::kIsBf16) {
+            const float2 fa = Pack2<T>::unpack(wa[j]), fb = Pack2<T>::unpack(wb[j]);
+            qa[m][4 * h + j] = Pack2<__half>::pack(fa.x, fa.y);
+            qb[m][4 * h + j] = Pack2<__half>::pack(fb.x, fb.y);
+          } else {
+            qa[m][4 * h + j] = wa[j];
+            qb[m][4 * h + j] = wb[j];
+          }
+        }
+      }
+    }
+  }
+  float m_run[2] = {-INFINITY, -INFINITY}, l_run[2] = {0.f, 0.f};
+  float o[VW][4];
+#pragma unroll
+  for (int n = 0; n < VW; ++n) { o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f; }
+
+  const uint8_t* kc = reinterpret_cast<const uint8_t*>(p.k_cache);
+  const uint8_t* vc = reinterpret_cast<const uint8_t*>(p.v_cache);
+  const int32_t* bt = p.block_table + static_cast<int64_t>(b) * p.max_blocks_per_seq;
+  auto row_offset = [&](int key) -> int64_t {  // byte offset of (key, kvh, dim 0)
+    const int bi = key / p.block_size;
+    const int in_blk = key - bi * p.block_size;
+    return ((static_cast<int64_t>(bt[bi]) * p.num_layers + p.layer_idx) * p.block_size + in_blk) *
+               (static_cast<int64_t>(p.Hkv) * D) + kvh * D;
+  };
+
+  auto issue_tile = [&](const int t0, uint4 (&kr)[4][MB], uint32_t (&vr)[2][4][VWORDS]) {
+#pragma unroll
+    for (int kg = 0; kg < 4; ++kg) {
+      const int key = t0 + kg * 8 + g;
+      const bool valid = key < k_end;
+      const int64_t off = valid ? row_offset(key) + 16 * t : 0;
+#pragma unroll
+      for (int m = 0; m < MB; ++m) kr[kg][m] = ld_stream_if(kc + off + 64 * m, valid);
+    }
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int key = t0 + 16 * s + 2 * t + (j & 1) + (j >> 1) * 8;
+        const bool valid = key < k_end;
+        const int64_t off = valid ? row_offset(key) + VW * g : 0;
+        if constexpr (VWORDS == 4) {
+          const uint4 r = ld_stream_if(vc + off, valid);
+          vr[s][j][0] = r.x; vr[s][j][1] = r.y; vr[s][j][2] = r.z; vr[s][j][3] = r.w;
+        } else {
+          const uint2 r = ld_stream8_if(vc + off, valid);
+          vr[s][j][0] = r.x; vr[s][j][1] = r.y;
+        }
+      }
+    }
+  };
+  // the two 16-key halves of a tile one after the other: the scores and probabilities of 16 keys are live at a time
+  auto compute_tile = [&](const int t0, const uint4 (&kr)[4][MB], const uint32_t (&vr)[2][4][VWORDS]) {
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      // ---- S = Q K^T (rows g, g+8; keys 16s + kg*8 + 2t, +1) ----
+      float sc[2][4];
+#pragma unroll
+      for (int kg = 0; kg < 2; ++kg) {
+        sc[kg][0] = sc[kg][1] = sc[kg][2] = sc[kg][3] = 0.f;
+#pragma unroll
+        for (int m = 0; m < MB; ++m) {
+          const uint4 kw = kr[2 * s + kg][m];
+          const uint32_t w[4] = {kw.x, kw.y, kw.z, kw.w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            mma_16816<__half>(sc[kg], qa[m][2 * j], qb[m][2 * j], qa[m][2 * j + 1], qb[m][2 * j + 1], widen2(w[j]),
+                              widen2(w[j] >> 16));
+        }
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const int key = t0 + 16 * s + kg * 8 + 2 * t + (e & 1);
+          sc[kg][e] = key < k_end ? sc[kg][e] * p.scale_log2 : -INFINITY;
+        }
+      }
+      // ---- online softmax for the two rows this lane holds ----
+      float pr[2][4];
+#pragma unroll
+      for (int r = 0; r < 2; ++r) {
+        float tmax = fmaxf(fmaxf(sc[0][2 * r], sc[0][2 * r + 1]), fmaxf(sc[1][2 * r], sc[1][2 * r + 1]));
+        tmax = fmaxf(tmax, __shfl_xor_sync(0xffffffffu, tmax, 1));
+        tmax = fmaxf(tmax, __shfl_xor_sync(0xffffffffu, tmax, 2));
+        const float m_new = fmaxf(m_run[r], tmax);
+        const float m_safe = (m_new == -INFINITY) ? 0.f : m_new;
+        const float corr = fast_exp2(m_run[r] - m_safe);
+        m_run[r] = m_new;
+        l_run[r] *= corr;
+#pragma unroll
+        for (int n = 0; n < VW; ++n) { o[n][2 * r] *= corr; o[n][2 * r + 1] *= corr; }
+#pragma unroll
+        for (int kg = 0; kg < 2; ++kg) {
+          pr[kg][2 * r] = fast_exp2(sc[kg][2 * r] - m_safe);
+          pr[kg][2 * r + 1] = fast_exp2(sc[kg][2 * r + 1] - m_safe);
+          l_run[r] += pr[kg][2 * r] + pr[kg][2 * r + 1];
+        }
+      }
+      // ---- O += P V ----
+      const uint32_t pa0 = Pack2<__half>::pack(pr[0][0], pr[0][1]), pa1 = Pack2<__half>::pack(pr[0][2], pr[0][3]);
+      const uint32_t pa2 = Pack2<__half>::pack(pr[1][0], pr[1][1]), pa3 = Pack2<__half>::pack(pr[1][2], pr[1][3]);
+#pragma unroll
+      for (int q4 = 0; q4 < VWORDS; ++q4) {
+        // bytes of keys (2t, 2t+1) and (2t+8, 2t+9), interleaved: [k0.b0, k1.b0, k0.b1, k1.b1] and [k0.b2, k1.b2, ...]
+        const uint32_t lo01 = __byte_perm(vr[s][0][q4], vr[s][1][q4], 0x5140);
+        const uint32_t hi01 = __byte_perm(vr[s][0][q4], vr[s][1][q4], 0x7362);
+        const uint32_t lo23 = __byte_perm(vr[s][2][q4], vr[s][3][q4], 0x5140);
+        const uint32_t hi23 = __byte_perm(vr[s][2][q4], vr[s][3][q4], 0x7362);
+        mma_16816<__half>(o[4 * q4 + 0], pa0, pa1, pa2, pa3, widen2(lo01), widen2(lo23));
+        mma_16816<__half>(o[4 * q4 + 1], pa0, pa1, pa2, pa3, widen2(lo01 >> 16), widen2(lo23 >> 16));
+        mma_16816<__half>(o[4 * q4 + 2], pa0, pa1, pa2, pa3, widen2(hi01), widen2(hi23));
+        mma_16816<__half>(o[4 * q4 + 3], pa0, pa1, pa2, pa3, widen2(hi01 >> 16), widen2(hi23 >> 16));
+      }
+    }
+  };
+  constexpr int STEP = GQA_WARPS * TILE;
+  {
+    uint4 krA[4][MB], krB[4][MB];
+    uint32_t vrA[2][4][VWORDS], vrB[2][4][VWORDS];
+    int t0 = k_begin + warp * TILE;
+    if (t0 < k_end) issue_tile(t0, krA, vrA);
+    for (; t0 < k_end; t0 += 2 * STEP) {
+      if (t0 + STEP < k_end) issue_tile(t0 + STEP, krB, vrB);
+      compute_tile(t0, krA, vrA);
+      if (t0 + 2 * STEP < k_end) issue_tile(t0 + 2 * STEP, krA, vrA);
+      if (t0 + STEP < k_end) compute_tile(t0 + STEP, krB, vrB);
+    }
+  }
+
+  // ---- combine: lanes of a row quad, then the warps of the CTA through shared memory ----
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 1);
+    l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 2);
+  }
+  __shared__ float sm_m[GQA_WARPS * 16];
+  __shared__ float sm_l[GQA_WARPS * 16];
+  __shared__ float sm_acc[GQA_WARPS * 16 * D];
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    const int row = g + 8 * r;
+    if (row < G) {
+      if (t == 0) { sm_m[warp * 16 + row] = m_run[r]; sm_l[warp * 16 + row] = l_run[r]; }
+#pragma unroll
+      for (int n = 0; n < VW; ++n) {
+        sm_acc[(warp * 16 + row) * D + VW * (2 * t) + n] = o[n][2 * r];
+        sm_acc[(warp * 16 + row) * D + VW * (2 * t + 1) + n] = o[n][2 * r + 1];
+      }
+    }
+  }
+  __syncthreads();
+  for (int idx = threadIdx.x; idx < G * D; idx += GQA_WARPS * 32) {
+    const int row = idx / D, d = idx - row * D;
+    float m = -INFINITY;
+#pragma unroll
+    for (int w = 0; w < GQA_WARPS; ++w) m = fmaxf(m, sm_m[w * 16 + row]);
+    const float m_safe = (m == -INFINITY) ? 0.f : m;
+    float l = 0.f, acc = 0.f;
+#pragma unroll
+    for (int w = 0; w < GQA_WARPS; ++w) {
+      const float c = fast_exp2(sm_m[w * 16 + row] - m_safe);
+      l = fmaf(sm_l[w * 16 + row], c, l);
+      acc = fmaf(sm_acc[(w * 16 + row) * D + d], c, acc);
+    }
+    const float out = l > 0.f ? acc / l * v_scale : 0.f;
+    const float lse = l > 0.f ? (m + log2f(l)) * kLn2 : -INFINITY;
+    const int h = kvh * G + row;
+    if (p.splits == 1) {
+      T* op = reinterpret_cast<T*>(p.o) + (static_cast<int64_t>(b) * p.Hq + h) * D + d;
+      if constexpr (Pack2<T>::kIsBf16) *op = __float2bfloat16_rn(out);
+      else *op = __float2half_rn(out);
+      if (d == 0 && p.lse != nullptr) p.lse[static_cast<int64_t>(b) * p.Hq + h] = lse;
+    } else {
+      const int64_t prow = (static_cast<int64_t>(b) * p.Hq + h) * p.splits + split;
+      p.part_o[prow * D + d] = out;
+      if (d == 0) p.part_lse[prow] = lse;
+    }
+  }
+}
+
+template <int D, typename T>
+int launch_decode(int G, const Params& p, float v_scale, cudaStream_t stream) {
+  dim3 grid(p.splits, p.Hkv, p.B);
+  if (G >= 3) {
+    decode_gqa_mma_kernel<D, T><<<grid, GQA_WARPS * 32, 0, stream>>>(p, G, v_scale);
+    B200_CUDA_OK(cudaGetLastError());
+    note_launch("fp8_decode_gqa_mma_kernel");
+  } else {
+    if (G == 1) decode_kernel<D, 1, T><<<grid, NUM_THREADS, 0, stream>>>(p, v_scale);
+    else decode_kernel<D, 2, T><<<grid, NUM_THREADS, 0, stream>>>(p, v_scale);
+    B200_CUDA_OK(cudaGetLastError());
+    note_launch("fp8_decode_kernel");
+  }
+  if (p.splits > 1) {
+    decode_reduce_kernel<D, T><<<p.B * p.Hq, D, 0, stream>>>(p.part_o, p.part_lse, p.o, p.lse, p.splits);
+    B200_CUDA_OK(cudaGetLastError());
+    note_launch("decode_reduce_kernel");
+  }
+  return B200_OK;
+}
+
+inline bool scale_ok(float s) { return s > 0.f && s <= 3.402823466e38f; }  // false for NaN, +-inf, 0 and negatives
+
+}  // namespace fp8
 }  // namespace decode
 }  // namespace b200
 
@@ -873,6 +1385,92 @@ int b200_kv_append(const void* key, const void* value, void* k_cache, void* v_ca
       max_blocks_per_seq, block_size, num_layers, layer_idx, capacity);
   B200_CUDA_OK(cudaGetLastError());
   note_launch("kv_append_kernel");
+  return B200_OK;
+}
+
+int b200_fa_decode_fp8(const void* q, const void* k_cache, const void* v_cache, void* o, float* lse, int B, int Hq, int Hkv,
+                       int D, const int32_t* context_lens, int max_context_len, float softmax_scale, int layout,
+                       const int32_t* block_table, int max_blocks_per_seq, int block_size, int num_layers, int layer_idx,
+                       int num_splits, void* workspace, int64_t workspace_bytes, float k_scale, float v_scale, int dtype,
+                       void* stream) {
+  using namespace b200;
+  B200_CHECK_ARG(q && k_cache && v_cache && o && context_lens, "decode_fp8: NULL pointer argument");
+  B200_CHECK_ARG(B > 0 && Hq > 0 && Hkv > 0 && Hq % Hkv == 0 && Hq / Hkv <= 16,
+                 "decode_fp8: bad B/Hq/Hkv = %d/%d/%d (Hq/Hkv must be 1 .. 16)", B, Hq, Hkv);
+  B200_CHECK_ARG(D == 64 || D == 128, "decode_fp8: head_dim %d unsupported (64, 128)", D);
+  B200_CHECK_ARG(dtype == B200_DTYPE_BF16 || dtype == B200_DTYPE_FP16, "decode_fp8: q dtype must be bf16 or fp16");
+  B200_CHECK_ARG(layout == B200_KV_CONTIGUOUS || layout == B200_KV_PAGED, "decode_fp8: unknown KV layout %d", layout);
+  if (layout != B200_KV_PAGED)
+    return set_error(B200_ERR_UNSUPPORTED, "decode_fp8: an FP8 cache exists in the paged layout only");
+  B200_CHECK_ARG(max_context_len > 0, "decode_fp8: max_context_len must be positive");
+  B200_CHECK_ARG(((uintptr_t)q & 15) == 0 && ((uintptr_t)k_cache & 15) == 0 && ((uintptr_t)v_cache & 15) == 0 &&
+                     ((uintptr_t)o & 15) == 0,
+                 "decode_fp8: pointers must be 16-byte aligned");
+  B200_CHECK_ARG(block_table != nullptr && block_size > 0 && max_blocks_per_seq > 0 && num_layers > 0 && layer_idx >= 0 &&
+                     layer_idx < num_layers,
+                 "decode_fp8: bad paged-cache arguments");
+  B200_CHECK_ARG(decode::fp8::scale_ok(k_scale) && decode::fp8::scale_ok(v_scale),
+                 "decode_fp8: k_scale and v_scale must be positive and finite (got %g, %g)", k_scale, v_scale);
+  const int splits = num_splits > 0 ? num_splits : b200_fa_decode_num_splits(B, Hq, Hkv, D, max_context_len);
+  decode::Params p;
+  p.q = q; p.k_cache = k_cache; p.v_cache = v_cache; p.o = o; p.lse = lse;
+  p.part_o = nullptr; p.part_lse = nullptr;
+  if (splits > 1) {
+    const int64_t need = b200_fa_decode_workspace_bytes(B, Hq, Hkv, D, max_context_len, splits);
+    if (workspace == nullptr || workspace_bytes < need)
+      return set_error(B200_ERR_WORKSPACE, "decode_fp8 workspace too small: need %lld bytes, got %lld", (long long)need,
+                       (long long)workspace_bytes);
+    p.part_o = static_cast<float*>(workspace);
+    p.part_lse = p.part_o + static_cast<int64_t>(B) * Hq * splits * D;
+  }
+  p.context_lens = context_lens; p.block_table = block_table;
+  p.B = B; p.Hq = Hq; p.Hkv = Hkv; p.splits = splits;
+  p.scale_log2 = softmax_scale * k_scale * decode::kLog2e;   // q . (byte * k_scale) = (q . byte) * k_scale
+  p.kv_batch_stride = 0; p.kv_token_stride = 0;
+  p.max_blocks_per_seq = max_blocks_per_seq; p.block_size = block_size; p.num_layers = num_layers;
+  p.layer_idx = layer_idx;
+  p.capacity = max_context_len < max_blocks_per_seq * block_size ? max_context_len : max_blocks_per_seq * block_size;
+  const int G = Hq / Hkv;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (D == 128) {
+    return dtype == B200_DTYPE_BF16 ? decode::fp8::launch_decode<128, __nv_bfloat16>(G, p, v_scale, s)
+                                    : decode::fp8::launch_decode<128, __half>(G, p, v_scale, s);
+  }
+  return dtype == B200_DTYPE_BF16 ? decode::fp8::launch_decode<64, __nv_bfloat16>(G, p, v_scale, s)
+                                  : decode::fp8::launch_decode<64, __half>(G, p, v_scale, s);
+}
+
+int b200_kv_append_fp8(const void* key, const void* value, void* k_cache, void* v_cache, int B, int n_tokens, int Hkv, int D,
+                       const int32_t* context_lens, const int32_t* block_table, int max_blocks_per_seq, int block_size,
+                       int num_layers, int layer_idx, float k_scale, float v_scale, int dtype, void* stream) {
+  using namespace b200;
+  B200_CHECK_ARG(key && value && k_cache && v_cache && context_lens, "kv_append_fp8: NULL pointer argument");
+  B200_CHECK_ARG(B > 0 && B <= 65535 && n_tokens > 0 && Hkv > 0, "kv_append_fp8: bad sizes B/n_tokens/Hkv = %d/%d/%d", B,
+                 n_tokens, Hkv);
+  B200_CHECK_ARG(D == 64 || D == 128, "kv_append_fp8: head_dim %d unsupported (64, 128)", D);
+  B200_CHECK_ARG(dtype == B200_DTYPE_BF16 || dtype == B200_DTYPE_FP16, "kv_append_fp8: key dtype must be bf16 or fp16");
+  B200_CHECK_ARG(((uintptr_t)key & 15) == 0 && ((uintptr_t)value & 15) == 0 && ((uintptr_t)k_cache & 15) == 0 &&
+                     ((uintptr_t)v_cache & 15) == 0,
+                 "kv_append_fp8: pointers must be 16-byte aligned");
+  B200_CHECK_ARG(block_table != nullptr && block_size > 0 && max_blocks_per_seq > 0 && num_layers > 0 && layer_idx >= 0 &&
+                     layer_idx < num_layers,
+                 "kv_append_fp8: bad paged-cache arguments");
+  B200_CHECK_ARG(decode::fp8::scale_ok(k_scale) && decode::fp8::scale_ok(v_scale),
+                 "kv_append_fp8: k_scale and v_scale must be positive and finite (got %g, %g)", k_scale, v_scale);
+  const dim3 grid(n_tokens, B);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  uint8_t* kd = static_cast<uint8_t*>(k_cache);
+  uint8_t* vd = static_cast<uint8_t*>(v_cache);
+  if (dtype == B200_DTYPE_BF16)
+    decode::fp8::kv_append_kernel<__nv_bfloat16><<<grid, 128, 0, s>>>(
+        static_cast<const __nv_bfloat16*>(key), static_cast<const __nv_bfloat16*>(value), kd, vd, context_lens, n_tokens,
+        Hkv * D, block_table, max_blocks_per_seq, block_size, num_layers, layer_idx, k_scale, v_scale);
+  else
+    decode::fp8::kv_append_kernel<__half><<<grid, 128, 0, s>>>(
+        static_cast<const __half*>(key), static_cast<const __half*>(value), kd, vd, context_lens, n_tokens, Hkv * D,
+        block_table, max_blocks_per_seq, block_size, num_layers, layer_idx, k_scale, v_scale);
+  B200_CUDA_OK(cudaGetLastError());
+  note_launch("fp8_kv_append_kernel");
   return B200_OK;
 }
 

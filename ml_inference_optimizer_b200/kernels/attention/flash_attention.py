@@ -363,10 +363,13 @@ class _HFAttentionAdapter(nn.Module):
                 attn = ops.flash_attn_fwd(q, k, v, causal=True, softmax_scale=inner.config.softmax_scale)
             else:
                 kc, vc = paged.get_physical_caches()
-                ops.kv_append(k[:, 0], v[:, 0], kc, vc, ctx_["context_lengths"], ctx_["block_tables"], self.layer_idx)
+                ks, vs = paged.layer_scales(self.layer_idx)
+                ops.kv_append(k[:, 0], v[:, 0], kc, vc, ctx_["context_lengths"], ctx_["block_tables"], self.layer_idx,
+                              k_scale=ks, v_scale=vs)
                 attn = ops.decode_attention(q[:, 0].contiguous(), kc, vc, ctx_["context_lengths"],
                                             softmax_scale=inner.config.softmax_scale, block_tables=ctx_["block_tables"],
-                                            layer_idx=self.layer_idx, max_context_len=ctx_.get("max_context_len")).unsqueeze(1)
+                                            layer_idx=self.layer_idx, max_context_len=ctx_.get("max_context_len"),
+                                            k_scale=ks, v_scale=vs).unsqueeze(1)
             out = inner.o_proj(attn.reshape(B, S, inner.hidden_size).to(orig))
             return (out,) + (None,) * (self.returns_tuple_len - 1)
         if cache is not None and hasattr(cache, "update"):

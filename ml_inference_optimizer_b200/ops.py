@@ -79,6 +79,25 @@ def _pad_head(t: torch.Tensor, width: int) -> torch.Tensor:
     return t if t.shape[-1] == width else torch.nn.functional.pad(t, (0, width - t.shape[-1]))
 
 
+#: element type of an FP8 KV cache (e4m3, max finite 448); the format is defined in include/b200_attn_mlp.h
+FP8 = torch.float8_e4m3fn
+
+
+def _fp8_cache(k_cache: torch.Tensor, v_cache: torch.Tensor, block_tables: Optional[torch.Tensor], k_scale: float,
+               v_scale: float) -> bool:
+    """True for an FP8 cache pair. Scales other than 1.0 belong to an FP8 cache; an FP8 cache is paged."""
+    fp8 = k_cache.dtype == FP8
+    if fp8 != (v_cache.dtype == FP8):
+        raise ValueError("k_cache and v_cache must both be FP8 or both 16-bit")
+    if not fp8:
+        if float(k_scale) != 1.0 or float(v_scale) != 1.0:
+            raise ValueError("k_scale / v_scale apply to an FP8 (torch.float8_e4m3fn) cache only")
+        return False
+    if block_tables is None:
+        raise NotImplementedError("an FP8 KV cache exists in the paged layout only: pass block_tables")
+    return True
+
+
 # --------------------------------------------------------------------------------------------------------
 # K1 prefill attention
 # --------------------------------------------------------------------------------------------------------
@@ -171,6 +190,8 @@ def paged_prefill_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: tor
         raise ValueError("expected q [B,Sq,Hq,D] and caches [num_blocks, L, block_size, Hkv, D]")
     B, Sq, Hq, D = q.shape
     num_blocks, num_layers, block_size, Hkv, Dk = k_cache.shape
+    if k_cache.dtype == FP8 or v_cache.dtype == FP8:
+        raise NotImplementedError("paged_prefill_attention reads 16-bit caches only: an FP8 cache is read by decode_attention")
     if Dk < D or k_cache.dtype != q.dtype or v_cache.dtype != q.dtype:
         raise ValueError("cache head_dim / dtype must match q")
     if Dk != D:   # a narrower head stored in a wider cache (cache_head_dim): zero columns behind q, the caller's scale
@@ -261,19 +282,22 @@ def _workspace(dev: torch.device, nbytes: int) -> Optional[torch.Tensor]:
 def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tensor, context_lens: torch.Tensor,
                      softmax_scale: Optional[float] = None, block_tables: Optional[torch.Tensor] = None,
                      layer_idx: int = 0, max_context_len: Optional[int] = None, num_splits: int = 0,
-                     return_lse: bool = False, out: Optional[torch.Tensor] = None):
+                     return_lse: bool = False, out: Optional[torch.Tensor] = None, k_scale: float = 1.0,
+                     v_scale: float = 1.0):
     """Single-token attention against a KV cache.
 
     q ``[B,Hq,D]``. Contiguous cache: k/v ``[B,S_max,Hkv,D]`` (``block_tables is None``). Paged cache: k/v
     ``[num_blocks, L, block_size, Hkv, D]`` + ``block_tables`` int32 ``[B,max_blocks]`` + ``layer_idx``.
     ``context_lens`` int32 ``[B]`` counts the valid keys (the appended token included).
+    A ``torch.float8_e4m3fn`` cache (paged only) holds K / ``k_scale`` and V / ``v_scale`` (``b200_fa_decode_fp8``).
     """
     dev = _require_cuda(q, k_cache, v_cache, context_lens, block_tables, out)
     if q.dim() != 3:
         raise ValueError(f"q must be [B,Hq,D], got {tuple(q.shape)}")
     B, Hq, D = q.shape
     dt = _dtype_code(q)
-    if k_cache.dtype != q.dtype or v_cache.dtype != q.dtype:
+    fp8 = _fp8_cache(k_cache, v_cache, block_tables, k_scale, v_scale)
+    if not fp8 and (k_cache.dtype != q.dtype or v_cache.dtype != q.dtype):
         raise ValueError("cache dtype must match q")
     if context_lens.dtype != torch.int32 or not context_lens.is_contiguous() or context_lens.numel() != B:
         raise ValueError("context_lens must be a contiguous int32 [B] tensor")
@@ -305,7 +329,7 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
     if Dk != D:   # a narrower head stored in a wider cache (cache_head_dim)
         scale = float(softmax_scale) if softmax_scale is not None else 1.0 / math.sqrt(D)
         res = decode_attention(_pad_head(q, Dk), k_cache, v_cache, context_lens, scale, block_tables, layer_idx, max_context_len,
-                               num_splits, return_lse)
+                               num_splits, return_lse, k_scale=k_scale, v_scale=v_scale)
         o = (res[0] if return_lse else res)[..., :D]
         if out is not None:
             out.copy_(o)
@@ -323,6 +347,13 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
         splits = num_splits if num_splits > 0 else lib.b200_fa_decode_num_splits(B, Hq, Hkv, D, max_context_len)
         ws_bytes = lib.b200_fa_decode_workspace_bytes(B, Hq, Hkv, D, max_context_len, splits)
         ws = _workspace(dev, ws_bytes)
+        if fp8:
+            rc = lib.b200_fa_decode_fp8(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), out.data_ptr(), _ptr(lse), B,
+                                        Hq, Hkv, D, context_lens.data_ptr(), max_context_len, scale, layout,
+                                        _ptr(block_tables), max_blocks, block_size, num_layers, int(layer_idx), splits,
+                                        _ptr(ws), ws_bytes, float(k_scale), float(v_scale), dt, _stream_ptr(dev))
+            check("b200_fa_decode_fp8", rc)
+            return (out, lse) if return_lse else out
         rc = lib.b200_fa_decode(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), out.data_ptr(), _ptr(lse), B, Hq,
                                 Hkv, D, context_lens.data_ptr(), max_context_len, scale, layout, kv_bs, kv_ts,
                                 _ptr(block_tables), max_blocks, block_size, num_layers, int(layer_idx), splits,
@@ -332,14 +363,23 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
 
 
 def kv_append(key: torch.Tensor, value: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tensor,
-              context_lens: torch.Tensor, block_tables: Optional[torch.Tensor] = None, layer_idx: int = 0) -> None:
-    """Write the new token's K,V ``[B,Hkv,D]`` into the cache at position ``context_lens[b]-1``."""
+              context_lens: torch.Tensor, block_tables: Optional[torch.Tensor] = None, layer_idx: int = 0,
+              k_scale: float = 1.0, v_scale: float = 1.0) -> None:
+    """Write the new token's K,V ``[B,Hkv,D]`` into the cache at position ``context_lens[b]-1``.
+
+    A ``torch.float8_e4m3fn`` cache (paged only) stores e4m3(K / ``k_scale``) and e4m3(V / ``v_scale``)
+    (``b200_kv_append_fp8``); it also takes ``[B,n,Hkv,D]`` rows, written to positions ``[context_lens[b]-n,
+    context_lens[b])`` (the prompt of a prefill)."""
     dev = _require_cuda(key, value, k_cache, v_cache, context_lens, block_tables)
-    if key.dim() != 3 or value.shape != key.shape:
+    fp8 = _fp8_cache(k_cache, v_cache, block_tables, k_scale, v_scale)
+    if fp8 and key.dim() == 4 and value.shape == key.shape:
+        B, n_tokens, Hkv, D = key.shape
+    elif key.dim() != 3 or value.shape != key.shape:
         raise ValueError(f"key / value must be [B,Hkv,D], got {tuple(key.shape)}, {tuple(value.shape)}")
-    B, Hkv, D = key.shape
+    else:
+        (B, Hkv, D), n_tokens = key.shape, 1
     _dtype_code(key)
-    if value.dtype != key.dtype or k_cache.dtype != key.dtype or v_cache.dtype != key.dtype:
+    if value.dtype != key.dtype or (not fp8 and (k_cache.dtype != key.dtype or v_cache.dtype != key.dtype)):
         raise ValueError("key, value and both caches must share a dtype")
     if context_lens.dtype != torch.int32 or not context_lens.is_contiguous() or context_lens.numel() != B:
         raise ValueError("context_lens must be a contiguous int32 [B] tensor")
@@ -368,6 +408,14 @@ def kv_append(key: torch.Tensor, value: torch.Tensor, k_cache: torch.Tensor, v_c
     if Dc != D:   # a narrower head stored in a wider cache (cache_head_dim): zero columns behind the new token's K, V
         key, value, D = _pad_head(key, Dc), _pad_head(value, Dc), Dc
     lib = _lib.load()
+    if fp8:
+        with torch.cuda.device(dev):
+            rc = lib.b200_kv_append_fp8(key.data_ptr(), value.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), B, n_tokens,
+                                        Hkv, D, context_lens.data_ptr(), block_tables.data_ptr(), max_blocks, block_size,
+                                        num_layers, int(layer_idx), float(k_scale), float(v_scale), _dtype_code(key),
+                                        _stream_ptr(dev))
+        check("b200_kv_append_fp8", rc)
+        return
     with torch.cuda.device(dev):
         rc = lib.b200_kv_append(key.data_ptr(), value.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), B, Hkv, D,
                                 context_lens.data_ptr(), KV_PAGED if paged else KV_CONTIGUOUS, kv_bs, kv_ts,
